@@ -5,6 +5,7 @@ for a complex transform, and ms/transform).
     python bench.py --gpus N --steps K --warmup W            # our CUDA path (libdfft.so)
     python bench.py --impl reference --gpus N --steps K ...  # CPU arm: the oracle port (scipy pocketfft)
     torchrun --nproc-per-node N ... bench.py --gpus N ...    # one rank per GPU, NCCL / NVLink peer stores
+    python bench.py ... --dump-outputs DIR                   # also save the last timed step's spectrum (seeded sample)
 
 A step is ONE forward complex-double 3D transform of the workload grid through the reference-shaped plan
 API (MPIcuFFT_Slab.execC2C).  Workload (weak scaling, 512^3 points per GPU — BASELINE configs[1] at N=1,
@@ -106,6 +107,26 @@ class ClockSampler:
             out["samples"] = len(sm)
         out["reasons"] = sorted(reasons)
         return out
+
+
+DUMP_VALUES = 1 << 21  # complex values written by --dump-outputs over all ranks: 32 MiB as float64 pairs
+
+
+def dump_outputs(path, out, osz, rank, world):
+    """--dump-outputs: the spectrum block that the last timed forward step left in `out`, as <path>/spectrum_rank<r>.npy,
+    float64 [n, 2] (real, imag).  A block of more than DUMP_VALUES / world values is sampled at fixed positions (the
+    sorted flat indices drawn by a seed-0 generator), so two builds with the same arguments compare value for value."""
+    import numpy as np
+    import torch
+
+    n = osz[0] * osz[1] * osz[2]
+    k = DUMP_VALUES // world
+    flat = out[:n]
+    if n > k:
+        idx = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+        flat = flat[torch.from_numpy(idx).to(flat.device)]
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, f"spectrum_rank{rank}.npy"), torch.view_as_real(flat).to(torch.float64).cpu().numpy())
 
 
 _CPU_INPUT = {}
@@ -325,7 +346,11 @@ def main(argv=None):
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-tune", action="store_true", help="keep the default overlapped schedule instead of measuring the candidates at plan time")
     ap.add_argument("--no-parity", action="store_true", help="skip the correctness checks in front of the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's output block (sampled above 2M values) to DIR/spectrum_rank<r>.npy")
     args = ap.parse_args(argv)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "dfft" else args.warmup
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -427,6 +452,8 @@ def main(argv=None):
     sampler = ClockSampler(local) if rank == 0 else None  # keeps sampling through the breakdown and e2e loops
     total_ms = timed(step, args.steps)
     plan.wait()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out, osz, rank, world)
     launches = plan.lastLaunchCount() * args.steps
     ms_step = total_ms / args.steps
     # inverse transform of the same grid (reported beside the headline; BASELINE config 1 names forward+inverse)

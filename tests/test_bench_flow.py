@@ -81,9 +81,9 @@ def _fake_dfft():
 
 
 @pytest.mark.parametrize("extra", [[], ["--transform", "r2c"], ["--no-e2e", "--no-cpu"], ["WORLD=8"], ["WORLD=8", "--decomp", "pencil", "--p1", "2", "--p2", "4", "--prec", "f32"],
-                                   ["WORLD=2", "--comm", "All2All", "--send", "Sync"]])
-def test_bench_single_gpu_flow_with_mocks(monkeypatch, capsys, extra):
-    extra = list(extra)
+                                   ["WORLD=2", "--comm", "All2All", "--send", "Sync"], ["--dump-outputs", "DUMP"]])
+def test_bench_single_gpu_flow_with_mocks(monkeypatch, capsys, tmp_path, extra):
+    extra = [str(tmp_path / "dump") if a == "DUMP" else a for a in extra]
     world = 1
     if extra and extra[0].startswith("WORLD="):
         world = int(extra.pop(0).split("=")[1])
@@ -116,6 +116,7 @@ def test_bench_single_gpu_flow_with_mocks(monkeypatch, capsys, extra):
     import importlib
     bench = importlib.import_module("bench")
     monkeypatch.setattr(bench, "ClockSampler", lambda idx: types.SimpleNamespace(stop=lambda: {"sm_mhz": 1900.0, "sm_max_mhz": 1965.0, "reasons": []}))
+    monkeypatch.setattr(bench, "DUMP_VALUES", 1000)  # below the 32^3 block: the sampled path
     monkeypatch.setattr(bench, "cpu_fft_sample", lambda shape, reps=1, cores=None: (0.5, 8, "mock sample", 7.5))
     monkeypatch.setattr(os.path, "exists", lambda p, _e=os.path.exists: False if p.endswith("libcufft_ref.so") else _e(p))
     if world > 1:
@@ -138,6 +139,10 @@ def test_bench_single_gpu_flow_with_mocks(monkeypatch, capsys, extra):
         assert len(nv) == (2 if "pencil" in extra else 1)
         assert line["cpu_baseline"] is None and line["config"]["send_method"] == ("Sync" if "Sync" in extra else "Streams")
         return
+    if "--dump-outputs" in extra:
+        import numpy as np
+        a = np.load(tmp_path / "dump" / "spectrum_rank0.npy")
+        assert a.dtype == np.float64 and a.shape == (1000, 2)
     for key in ("bound", "achieved", "peak", "unit", "frac", "traffic"):
         assert key in line["roofline"]
     if "--no-e2e" not in extra:
